@@ -2,7 +2,9 @@
 (oracle/_ref/liboracle_ref_{fixed,float}.so = /root/reference/source/ImgDecode.cpp built unmodified)
 on small seeded JPEGs.  Run in the build container (needs /root/reference); the .npz files it
 writes are committed so the oracle port and the CUDA path can be checked where the reference is
-absent.  Usage: python tests/golden/make_golden.py
+absent.  It also stores, in ref_outputs.json.gz, what the compiled reference computes for the tests that compare with it
+(record_reference() of each module in REF_MODULES).
+Usage: python tests/golden/make_golden.py [ref_outputs]     (ref_outputs: only ref_outputs.json.gz)
 """
 import io
 import os
@@ -13,6 +15,9 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.dirname(HERE)); sys.path.insert(0, os.path.dirname(os.path.dirname(HERE)))
 from oracle_util import Oracle, build_oracles      # noqa: E402
 import jpeg_cases as JC                            # noqa: E402
+import ref_golden as RG                            # noqa: E402
+
+REF_MODULES = ("test_oracle", "test_gpu_parity", "test_gpu_preview", "test_gpu_detail", "test_tiff_export")
 
 
 def fixtures():
@@ -46,5 +51,19 @@ def main():
         print(name, len(j), "bytes ->", os.path.getsize(os.path.join(HERE, name + ".npz")), "bytes npz")
 
 
+def ref_outputs():
+    import importlib
+    build_oracles()
+    out = {}
+    for m in REF_MODULES:
+        rec = importlib.import_module(m).record_reference(Oracle)
+        assert not set(rec) & set(out), m
+        out.update(rec)
+    RG.save(out)
+    print(len(out), "entries ->", os.path.getsize(RG.PATH), "bytes", RG.PATH)
+
+
 if __name__ == "__main__":
-    main()
+    if sys.argv[1:] != ["ref_outputs"]:
+        main()
+    ref_outputs()

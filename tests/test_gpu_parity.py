@@ -6,6 +6,7 @@ import numpy as np
 import pytest
 
 import jpeg_cases as JC
+import ref_golden as RG
 from oracle_util import Oracle, ref_available
 
 pytestmark = pytest.mark.gpu
@@ -158,17 +159,15 @@ def _damaged_cases(cases):
 
 @pytest.mark.parametrize("huff", [0, 1, 2], ids=["auto", "warp", "lane"])
 def test_damaged_scans_match_the_reference(built, cases, huff):
-    """Damaged scans, single-image drop-in: every output buffer AND every error line equal to the compiled reference's —
+    """Damaged scans, single-image drop-in: every output buffer AND every error line equal to the compiled reference's
+    (tests/golden/ref_outputs.json.gz) —
     its one-bit resynchronisation (ImgDecode.cpp:1166-1187), stray-marker handling (:1486-1561, 1683-1706), lazy restarts
     (:1644-1680), underflowing blocks (:1737-1760), the one-MCU-per-row tail after an overread (:3621-3625) and the
     nErrMaxDecodeScan cap (:1100-1110)."""
-    if not ref_available("fixed"):
-        pytest.skip("needs the compiled reference (oracle/_ref)")
     from jpegsnoop_b200 import CimgDecode
-    orc = Oracle("ref_fixed")
     dec = CimgDecode(idct_fixedpt=True, huff_kernel=huff, idct_kernel=0)
     for name, (j, ovl) in _damaged_cases(cases).items():
-        want = orc.decode(j, overlays=ovl); want_lines = orc.err_lines()
+        want = RG.get_decoded(f"damaged/{name}"); want_lines = RG.get(f"damaged/{name}/err_lines")
         dec.L.jsimg_overlay_remove_all(dec.h)
         keep = []
         for off, data in ovl:
@@ -178,27 +177,21 @@ def test_damaged_scans_match_the_reference(built, cases, huff):
         bad = JC.compare(want, got)
         assert not bad, f"{name}: mismatch in {bad}"
         assert np.array_equal(np.asarray(want.stats)[10:12], np.asarray(got.stats)[10:12]), (name, want.stats, got.stats)     # m_nRestartRead, m_bScanBad
-        got_lines = dec.log_lines(3)
-        assert got_lines == want_lines, (name, len(got_lines), len(want_lines), [(a, b) for a, b in zip(got_lines, want_lines) if a != b][:3])
+        diff = RG.lines_diff(want_lines, dec.log_lines(3))
+        assert not diff, (name, diff)
 
 
 def test_damaged_images_in_a_batch_match_the_reference(built, cases):
     """The same in one batch next to healthy images: the damaged ones carry JSGPU_ST_EXACT, their outputs are the reference's,
     their neighbours are untouched; the error-line count comes back through jsgpu_batch_errors."""
-    if not ref_available("fixed"):
-        pytest.skip("needs the compiled reference (oracle/_ref)")
     from jpegsnoop_b200 import BatchDecoder
-    orc = Oracle("ref_fixed")
-    dmg = {k: v for k, v in _damaged_cases(cases).items() if not v[1]}
-    names = ["ok0"] + list(dmg) + ["ok1"]
-    jpegs = [cases[2][1]] + [v[0] for v in dmg.values()] + [cases[1][1]]
+    names, jpegs = _damaged_batch(cases)
     WHAT = ("geom", "pix_y", "pix_cb", "pix_cr", "dib", "mcu_map", "blk_dc", "dht_histo")
     for dc_only in (False, True):
-        o = Oracle("ref_fixed", decode_ac=not dc_only)
         bd = BatchDecoder(huff_kernel=0, idct_kernel=0, decode_ac=not dc_only)
         bd.set_batch(jpegs); bd.decode(); bd.sync()
         for i, (name, j) in enumerate(zip(names, jpegs)):
-            want = o.decode(j); got = bd.fetch(i)
+            want = RG.get_decoded(f"damaged_batch/{dc_only}/{name}"); got = bd.fetch(i)
             assert not JC.compare(want, got, what=WHAT), (name, dc_only)
             if name.startswith("ok"):
                 assert got.status == 0, (name, hex(got.status))
@@ -206,6 +199,11 @@ def test_damaged_images_in_a_batch_match_the_reference(built, cases):
                 assert got.status & 0x40000000, (name, hex(got.status))
                 e = bd.scan_errors(i)
                 assert e.nerr_lines == want.nerr and e.scan_bad == int(want.stats[11]), (name, e.nerr_lines, want.nerr)
+
+
+def _damaged_batch(cases):
+    dmg = {k: v for k, v in _damaged_cases(cases).items() if not v[1]}
+    return ["ok0"] + list(dmg) + ["ok1"], [cases[2][1]] + [v[0] for v in dmg.values()] + [cases[1][1]]
 
 
 @pytest.mark.parametrize("nrep", [1, 2], ids=["single_stream_15", "chunked_30"])
@@ -334,3 +332,20 @@ def test_unsupported_images_in_a_batch_are_skipped(built, cases):
     for i, (nm, j) in enumerate(zip(names, jpegs)):
         if nm == "ok":
             assert not JC.compare(orc.decode(j), bd.fetch(i), what=("pix_y", "dib", "mcu_map")), i
+
+
+def record_reference(orc):
+    """What the compiled reference computes for the damaged-scan tests above (tests/golden/make_golden.py stores it)."""
+    out = {}
+    cases = JC.small_cases()
+    ref = orc("ref_fixed")
+    for name, (j, ovl) in _damaged_cases(cases).items():
+        out[f"damaged/{name}"] = RG.decoded(ref.decode(j, overlays=ovl)); out[f"damaged/{name}/err_lines"] = RG.lines(ref.err_lines())
+    ref.close()
+    names, jpegs = _damaged_batch(cases)
+    for dc_only in (False, True):
+        o = orc("ref_fixed", decode_ac=not dc_only)
+        for name, j in zip(names, jpegs):
+            out[f"damaged_batch/{dc_only}/{name}"] = RG.decoded(o.decode(j))
+        o.close()
+    return out
